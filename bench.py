@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- learner updates/sec of the Rainbow hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C3|C4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C3|C4] [--dump-outputs DIR]
 
 One step = `dqn.reset_noise(); dqn.learn(mem)` (reference main.py:150-151,163-164) on synthetic 84x84x4
 transitions.  N=1 workload = BASELINE.json configs[1] ("C2": 1M-transition replay in HBM, batch 32, 51
@@ -238,7 +238,7 @@ def reference_arm(opts, cfg, rank):
     per_step = 1  # one update (preceded by its 4 appends) per bench "step", exactly like our arm's e2e step
     ups, dt, threads, total, kind, sample, _ = cpu_arm(cfg, opts.steps * per_step, min(5, max(3, opts.warmup)), budget_s=150)
     line = {"impl": "reference", "metric": "learner updates/sec (batch32, 1M buffer, 51 atoms)", "value": ups,
-            "unit": "updates/s", "n_gpus": opts.gpus, "steps": opts.steps, "warmup": opts.warmup,
+            "unit": "updates/s", "n_gpus": opts.gpus, "steps": total, "warmup": opts.warmup,   # the 150 s budget may stop it early
             "ms_per_step": 1e3 * dt / total, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "gpu_launches": 0,
             "config": workload_config(opts.config, cfg, opts.gpus),
@@ -312,6 +312,32 @@ def kernel_source_sha(name):
     return csrc_sha256(sorted(KERNEL_SOURCES.get(name, ["rb_kernels.cu"]) + ["rb_internal.cuh"]))
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def last_step_outputs(agent, mem):
+    """What the last `reset_noise(); learn(mem)` left its caller, as host arrays: the per-sample losses, the tree indices
+    of the batch and the priorities written back for them, and every online-net parameter after the optimiser step
+    (6.9 M floats at C2 / C4)."""
+    import torch
+    idx = mem._last.tree_idx
+    out = {"loss": agent.last_loss, "tree_idx": idx.to(torch.float64), "priority": mem.transitions.tree[idx]}
+    out.update(("param." + name, p) for name, p in agent.online_net.named_parameters())
+    return {k: v.detach().cpu().numpy() for k, v in out.items()}
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: DIR/<name>.npy for every array (float32, or float64 for the indices)."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"dumped {len(arrays)} arrays ({total / 1e6:.1f} MB) of the last timed step to {directory}")
+
+
 def ours(opts, cfg, rank, world, local):
     import torch
 
@@ -322,7 +348,13 @@ def ours(opts, cfg, rank, world, local):
 
     torch.backends.cudnn.allow_tf32 = False        # the reference computes in true fp32
     torch.backends.cuda.matmul.allow_tf32 = False
-    torch.backends.cudnn.benchmark = True
+    # The conv algorithms cuDNN picks by timing for these shapes accumulate in a run-dependent order, and the prioritized
+    # replay turns such last-bit differences into different batches within a few hundred updates.  A run whose outputs
+    # are dumped therefore uses cuDNN's deterministic algorithms (heuristic choice): it reproduces bit for bit, and is
+    # slower (B200 at 1000 W, C2: 485 against 323 us per update).
+    deterministic = bool(opts.dump_outputs)
+    torch.backends.cudnn.benchmark = not deterministic
+    torch.backends.cudnn.deterministic = deterministic
     dev = torch.device("cuda", local)
     torch.cuda.set_device(dev)
     torch.manual_seed(shard_seed(0, rank))
@@ -404,6 +436,8 @@ def ours(opts, cfg, rank, world, local):
     # ---- value: inputs resident in HBM, K updates --------------------------------------------------
     ms_value = timed(lambda i: step(), K)
     log(f"value region: {ms_value / K:.3f} ms/step")
+    if opts.dump_outputs and rank == 0:   # before the e2e region below moves the parameters and the tree on
+        dump_outputs(opts.dump_outputs, last_step_outputs(agent, mem))
     # ---- e2e: public API with host frames ------------------------------------------------------------
     host_frames = [torch.rand(4, 84, 84).pin_memory() for _ in range(8)]
     loss_host = [torch.empty(B, dtype=torch.float32).pin_memory() for _ in range(2)]
@@ -445,7 +479,7 @@ def ours(opts, cfg, rank, world, local):
     agent.use_cuda_graph = False
     for _ in range(3):
         step()
-    timed_steps = min(K, 100)
+    timed_steps = min(K, 100)   # the library keeps events for 2048 launches per kernel id (PROF_SLOTS): up to 20 per step fit
     with _lib.KernelTimer() as kt:
         for i in range(timed_steps):
             for j in range(REPLAY_FREQUENCY if i % 10 == 0 else 0):
@@ -470,8 +504,8 @@ def ours(opts, cfg, rank, world, local):
                 a2.reset_noise()
                 a2.learn(mem)
 
-            ms_tf32 = timed(step_tf32, 100)
-            tf32_ctx = {"ms_per_step": ms_tf32 / 100, "value": 100 / (ms_tf32 * 1e-3), "unit": "updates/s",
+            ms_tf32 = timed(step_tf32, K)
+            tf32_ctx = {"ms_per_step": ms_tf32 / K, "value": K / (ms_tf32 * 1e-3), "unit": "updates/s",
                         "what": "Agent(args.tf32=True): cuDNN may use TF32 tensor-core kernels for the conv body (heads unchanged); outside "
                                 "the 1e-5 parity bar, reported for context only"}
         finally:
@@ -553,6 +587,9 @@ def ours(opts, cfg, rank, world, local):
             "clocks": clocks, "roofline": roofline}
     if tf32_ctx is not None:
         line["tf32_conv_context"] = tf32_ctx
+    if deterministic:
+        line["dump_outputs"] = {"dir": opts.dump_outputs, "cudnn": "deterministic algorithms, heuristic choice: reproducible "
+                                                                    "outputs, slower than a run without --dump-outputs"}
     if world == 1 and not opts.no_cpu_baseline:
         del agent, mem, tr                                  # give the 7 GB of HBM back before the reference's GPU leg
         torch.cuda.empty_cache()
@@ -604,7 +641,13 @@ def main():
     ap.add_argument("--nccl", action="store_true", help="N>1: NCCL all-reduce + replicated Adam (no peer-memory optimiser)")
     ap.add_argument("--profile-steps", type=int, default=0, help="run this many steps inside cudaProfilerStart/Stop and exit")
     ap.add_argument("--profile-mode", default="graph", choices=["graph", "eager", "e2e"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (losses, batch tree indices, priorities "
+                         "written back, online-net parameters) as DIR/<name>.npy; inputs are seeded and cuDNN runs its "
+                         "deterministic algorithms, so two builds compare output for output (the timing is then slower)")
     opts = ap.parse_args()
+    if opts.dump_outputs and (opts.impl != "ours" or opts.profile_steps):
+        ap.error("--dump-outputs needs --impl ours and no --profile-steps")
     cfg = CONFIGS[opts.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
