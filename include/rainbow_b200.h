@@ -73,7 +73,7 @@ enum {
   RB_K_TREE_UPDATE = 0, RB_K_TREE_FIND, RB_K_TREE_SAMPLE, RB_K_GATHER, RB_K_ITER_STATES, RB_K_APPEND, RB_K_C51,
   RB_K_NOISY_RESAMPLE, RB_K_NOISY_COMPOSE, RB_K_SQNORM, RB_K_CLIP_ADAM, RB_K_HEAD_FC1, RB_K_HEAD_FC2, RB_K_HEAD_LOGITS,
   RB_K_HEAD_WGRAD2, RB_K_HEAD_DH, RB_K_HEAD_BWD1, RB_K_NOISE_FACTORS, RB_K_C51_DUELING, RB_K_BIAS_GRAD, RB_K_Q_VALUES,
-  RB_K_HEAD_REDUCE1, RB_K_CONV_WGRAD, RB_KERNEL_COUNT
+  RB_K_HEAD_REDUCE1, RB_K_CONV_WGRAD, RB_K_CONV_FWD, RB_KERNEL_COUNT
 };
 
 int rb_abi_version(void);
@@ -256,6 +256,16 @@ int rb_bias_grad(const float* grad_out, int B, int C, int HW, float* out, rb_str
 int rb_conv_wgrad_scratch_elems(int B, int IC, int IH, int OC, int K, int stride);
 int rb_conv_wgrad(const float* grad_out, const float* input, int B, int IC, int IH, int IW, int OC, int K, int stride,
                   float* partials, float* out, float* bias_out, rb_stream_t stream);
+
+/* model.py:55-63, one conv layer of the network body and the ReLU after it:
+ * out[b][oc][oy][ox] = max(0, bias[oc] + sum_{ic,ky,kx} weight[oc][ic][ky][kx] * input[b][ic][oy*stride+ky][ox*stride+kx])
+ * for a square K x K kernel without padding, dilation or groups.  input float32 [B][IC][IH][IW], weight float32
+ * [OC][IC][K][K], bias float32 [OC], out float32 [B][OC][OH][OW] (OH = (IH-K)/stride + 1), all contiguous.
+ * Runs on the tensor cores as an error-compensated TF32 product (fp32-equivalent results whatever torch's allow_tf32 says),
+ * one launch, fixed summation order (deterministic).  (K, stride) in {(8,4), (4,2), (3,1), (5,5)} and OC % 32 == 0 are
+ * instantiated; other shapes return RB_ERR_RANGE without launching anything. */
+int rb_conv_forward(const float* input, const float* weight, const float* bias, int B, int IC, int IH, int IW, int OC, int K,
+                    int stride, float* out, rb_stream_t stream);
 
 /* rb_c51_loss_grad fed by the fused heads: z_online has 2B rows (s then s'), z_target B rows (s');
  * returns loss[B] and dz[B][atoms*(1+actions)] = d mean(w*loss) / d (z_value | z_advantage) of the online(s) rows

@@ -54,6 +54,7 @@ SIGNATURES = {
     "rb_bias_grad": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),
     "rb_conv_wgrad_scratch_elems": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32]),
     "rb_conv_wgrad": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
+    "rb_conv_forward": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "rb_c51_dueling_loss_grad": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _i32,
                                            _vp, _vp, _vp, _vp, _vp]),
     "rb_noisy_compose": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp]),
@@ -118,7 +119,7 @@ def stream():
 
 KERNEL_IDS = ["tree_update", "tree_find", "tree_sample", "gather", "iter_states", "append", "c51", "noisy_resample",
               "noisy_compose", "sqnorm", "clip_adam", "head_fc1", "head_fc2", "head_logits", "head_wgrad2", "head_dh",
-              "head_bwd1", "noise_factors", "c51_dueling", "bias_grad", "q_values", "head_reduce1", "conv_wgrad"]  # order of the enum in include/rainbow_b200.h
+              "head_bwd1", "noise_factors", "c51_dueling", "bias_grad", "q_values", "head_reduce1", "conv_wgrad", "conv_fwd"]  # order of the enum in include/rainbow_b200.h
 
 
 class KernelTimer:

@@ -141,8 +141,9 @@ class Agent:
         if self.device.type != "cuda":
             raise _lib.RainbowB200Error(f"rainbow_b200.Agent needs a CUDA device, got '{self.device}' (no CPU fallback)")
         # Precision policy (documented switch, default = the reference's arithmetic): the learner computes in true fp32.
-        # `args.tf32 = True` lets cuDNN / cuBLAS use TF32 tensor cores for the conv body (north star: "tensor cores only
-        # there"); the parity tests and bench.py run with the default.  torch keeps these flags per process, so the
+        # `args.tf32 = True` lets cuDNN / cuBLAS use TF32 tensor cores for the conv backward and the autograd fallback
+        # (features()); the own conv forward is fp32-accurate either way.  The parity tests and bench.py run with the
+        # default.  torch keeps these flags per process, so the
         # Agent sets them: what is measured is what ships.
         self.tf32 = bool(getattr(args, "tf32", False))
         torch.backends.cudnn.allow_tf32 = self.tf32
@@ -228,7 +229,7 @@ class Agent:
         self.online_net.reset_noise()
 
     def q_select(self, states, q_out=None):
-        """Greedy action and its value for a batch of states [N, history, 84, 84] (device): conv body (cuDNN), fused
+        """Greedy action and its value for a batch of states [N, history, 84, 84] (device): conv body (rb_conv_forward), fused
         noisy dueling head, then rb_q_values -- softmax over atoms, expectation over the support (agent.py:55) and the
         arg-max / max over actions in one launch.  Returns device tensors (actions int64[N], values float32[N]); nothing
         synchronises.  Falls back to plain torch ops for head shapes the fused kernels do not cover."""

@@ -990,6 +990,187 @@ k_conv_wgrad_reduce(const float* __restrict__ part, int n_part, int n_w, int n_b
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Conv body forward, one layer: y[b][oc][oy][ox] = relu(bias[oc] + sum_{ic,ky,kx} W[oc][ic][ky][kx] * x[b][ic][oy*S+ky][ox*S+kx])
+// (model.py:55-63, no padding, square kernel) as an implicit GEMM on the warp-level tensor-core path with an error-
+// compensated TF32 product (three MMAs per product as in k_head_bwd1; fp32-equivalent results, see tf32_split_rn below):
+// D[oc][p] = W[oc][k] x X[k][p], k = (ic, ky, kx).
+// grid = (bands of output rows, OC / 32, samples): a CTA owns 32 output channels of one band of one sample.  It stages the
+// input rows its band touches (all channels) and its 32 weight rows in shared memory with every copy in flight at once,
+// then warp work units (2 n8 pixel tiles x both m16 channel tiles, one slice of the k steps) run mma.sync.m16n8k8 with the
+// A operand (W) split into hi / lo once per k step and reused over the unit's two pixel tiles, and the B operand gathered
+// from the staged input through a per-k offset table.  The k slices of a pixel group land in separate shared buffers that
+// the epilogue sums in slice order (deterministic, no atomics), then adds the bias, applies the ReLU and writes the band's
+// rows coalesced.  These layers are latency bound at 32 / 64 rows, not arithmetic bound: the tiling exists to put a few
+// hundred CTAs on the machine, each with a short serial chain.
+// ------------------------------------------------------------------------------------------------
+// Numerics: tf32_split's truncated hi leaves lo with up to 13 significant bits, which the MMA truncates to TF32 again
+// (2^-21 relative per product), and one accumulator chained through ~100 MMAs adds the tensor core's inexact internal
+// accumulation step after step: measured 3.8e-6 max error on conv 0 against 0.9e-6 for cuDNN's fp32 kernel.  Here hi is
+// rounded to nearest (|lo| <= 2^-12 |v|, so lo's own TF32 truncation costs <= 2^-23) and each k step's three MMAs start from
+// zero and are added to the fp32 accumulator with an IEEE add.
+__device__ __forceinline__ void tf32_split_rn(float v, uint32_t& hi, uint32_t& lo) {
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hi) : "f"(v));
+  lo = __float_as_uint(__fsub_rn(v, __uint_as_float(hi)));
+}
+
+constexpr int CF_T = 256;           // threads per CTA
+constexpr int CF_WARPS = CF_T / 32;
+constexpr int CF_OC = 32;           // output channels per CTA (two m16 tiles)
+constexpr int CF_MAX_BAND = 5;      // output rows per band at most
+
+struct ConvFwdCfg {
+  int OH, OW, RB, bands, in_rows, npx, groups, ksplit, kdim, kpad, nk, ldw, ldr, slab;
+  size_t smem;
+};
+
+ConvFwdCfg conv_fwd_cfg(int IC, int IH, int IW, int K, int S) {
+  ConvFwdCfg c;
+  c.OH = (IH - K) / S + 1;
+  c.OW = (IW - K) / S + 1;
+  const int nb = (c.OH + CF_MAX_BAND - 1) / CF_MAX_BAND;
+  c.RB = (c.OH + nb - 1) / nb;                          // balanced bands: 20 -> 4 x 5, 9 -> 5 + 4, 7 -> 4 + 3, 16 -> 4 x 4
+  c.bands = (c.OH + c.RB - 1) / c.RB;
+  c.in_rows = (c.RB - 1) * S + K;
+  c.npx = c.RB * c.OW;                                  // pixels of a full band
+  c.groups = ((c.npx + 7) / 8 + 1) / 2;                 // warp units along the pixels: two n8 tiles each
+  c.kdim = IC * K * K;
+  c.kpad = (c.kdim + 7) & ~7;
+  c.nk = c.kpad / 8;
+  c.ksplit = CF_WARPS / c.groups;
+  if (c.ksplit < 1) c.ksplit = 1;
+  if (c.ksplit > c.nk) c.ksplit = c.nk;
+  c.ldw = ((c.kpad + 31) & ~31) + 4;                    // = 4 (mod 32): conflict-free A fragment loads
+  c.ldr = c.groups * 16 + 4;                            // partial buffer row stride (pixels)
+  c.slab = (IC * c.in_rows * IW + 3) & ~3;
+  c.smem = ((size_t)c.slab + (size_t)CF_OC * c.ldw + (size_t)c.ksplit * CF_OC * c.ldr + (size_t)c.kpad) * sizeof(float);
+  return c;
+}
+
+template <int K, int S>
+__global__ void __launch_bounds__(CF_T)
+k_conv_fwd(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias, int IC, int IH, int IW,
+           int OC, const ConvFwdCfg c, float* __restrict__ y) {
+  extern __shared__ __align__(16) float cf_smem[];
+  float* xs = cf_smem;                                            // [IC][in_rows][IW]   input rows of the band
+  float* ws = xs + c.slab;                                        // [32][ldw]           weight rows of the CTA's channels
+  float* red = ws + (size_t)CF_OC * c.ldw;                        // [ksplit][32][ldr]   partial tiles of the k slices
+  int* koff = reinterpret_cast<int*>(red + (size_t)c.ksplit * CF_OC * c.ldr);   // [kpad]  slab offset of k = (ic, ky, kx)
+  const int tid = threadIdx.x, band = blockIdx.x, oc0 = blockIdx.y * CF_OC, b = blockIdx.z;
+  const int y0 = band * c.RB, rows = min(c.RB, c.OH - y0), npx = rows * c.OW;
+  const int have_rows = min(c.in_rows, IH - y0 * S);
+  const int xs_ld = c.in_rows * IW;
+
+  // ---- staging: input slab and weight rows, all copies in flight at once ----
+  const float* xsrc = x + ((size_t)b * IC * IH + (size_t)y0 * S) * IW;
+  const int chunk = have_rows * IW;                               // contiguous floats per channel
+  if ((IW & 3) == 0 && ((uintptr_t)x & 15) == 0) {
+    const int q = chunk >> 2;
+    for (int i = tid; i < IC * q; i += CF_T) {
+      const int ic = i / q, j = i - ic * q;
+      cp_async16(xs + ic * xs_ld + 4 * j, xsrc + (size_t)ic * IH * IW + 4 * j);
+    }
+  } else {
+    for (int i = tid; i < IC * chunk; i += CF_T) {
+      const int ic = i / chunk, j = i - ic * chunk;
+      cp_async4(xs + ic * xs_ld + j, xsrc + (size_t)ic * IH * IW + j);
+    }
+  }
+  const float* wsrc = w + (size_t)oc0 * c.kdim;
+  if ((c.kdim & 3) == 0 && ((uintptr_t)w & 15) == 0) {
+    const int q = c.kdim >> 2;
+    for (int i = tid; i < CF_OC * q; i += CF_T) {
+      const int r = i / q, j = i - r * q;
+      cp_async16(ws + r * c.ldw + 4 * j, wsrc + (size_t)r * c.kdim + 4 * j);
+    }
+  } else {
+    for (int i = tid; i < CF_OC * c.kdim; i += CF_T) {
+      const int r = i / c.kdim, j = i - r * c.kdim;
+      cp_async4(ws + r * c.ldw + j, wsrc + (size_t)r * c.kdim + j);
+    }
+  }
+  // k padding (kdim % 8 != 0): zero weights, offset 0 (any finite staged value times zero)
+  for (int i = tid; i < CF_OC * (c.kpad - c.kdim); i += CF_T) {
+    const int r = i / (c.kpad - c.kdim), j = c.kdim + i % (c.kpad - c.kdim);
+    ws[r * c.ldw + j] = 0.0f;
+  }
+  for (int k = tid; k < c.kpad; k += CF_T) {
+    const int ic = k / (K * K), r = k - ic * (K * K), ky = r / K, kx = r - ky * K;
+    koff[k] = (k < c.kdim) ? ic * xs_ld + ky * IW + kx : 0;
+  }
+  cp_async_wait_all();
+  __syncthreads();
+
+  // ---- products: warp unit u = (pixel group u % groups, k slice u / groups) ----
+  const int warp = tid >> 5, lane = tid & 31, gid = lane >> 2, tig = lane & 3;
+  const int units = c.groups * c.ksplit, per = (c.nk + c.ksplit - 1) / c.ksplit;
+  for (int u = warp; u < units; u += CF_WARPS) {
+    const int grp = u % c.groups, ks = u / c.groups;
+    float acc[2][2][4];   // [m tile][n tile][C fragment]
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+#pragma unroll
+      for (int j = 0; j < 2; ++j)
+#pragma unroll
+        for (int q = 0; q < 4; ++q) acc[i][j][q] = 0.0f;
+    int poff[2];
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {   // B fragment column (pixel) of this lane in pixel tile j; pixels past the band read offset 0
+      const int p = grp * 16 + 8 * j + gid;
+      const int oy = p / c.OW, ox = p - oy * c.OW;
+      poff[j] = (p < npx) ? oy * S * IW + ox * S : 0;
+    }
+    const int s_begin = ks * per, s_end = min(c.nk, s_begin + per);
+    for (int s = s_begin; s < s_end; ++s) {
+      const int k0 = 8 * s;
+      uint32_t ahi[2][4], alo[2][4];
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const float* a = ws + (16 * i) * c.ldw + k0;
+        tf32_split_rn(a[gid * c.ldw + tig], ahi[i][0], alo[i][0]);
+        tf32_split_rn(a[(gid + 8) * c.ldw + tig], ahi[i][1], alo[i][1]);
+        tf32_split_rn(a[gid * c.ldw + tig + 4], ahi[i][2], alo[i][2]);
+        tf32_split_rn(a[(gid + 8) * c.ldw + tig + 4], ahi[i][3], alo[i][3]);
+      }
+      const int ko0 = koff[k0 + tig], ko1 = koff[k0 + tig + 4];
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        uint32_t bhi[2], blo[2];
+        tf32_split_rn(xs[ko0 + poff[j]], bhi[0], blo[0]);
+        tf32_split_rn(xs[ko1 + poff[j]], bhi[1], blo[1]);
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {   // D = Alo*Bhi + Ahi*Blo + Ahi*Bhi (the order of mma3_block), then acc += D
+          float d[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+          mma_tf32(d, alo[i], bhi);
+          mma_tf32(d, ahi[i], blo);
+          mma_tf32(d, ahi[i], bhi);
+#pragma unroll
+          for (int q = 0; q < 4; ++q) acc[i][j][q] += d[q];
+        }
+      }
+    }
+    float* dst = red + (size_t)ks * CF_OC * c.ldr + grp * 16;
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+#pragma unroll
+      for (int j = 0; j < 2; ++j)
+#pragma unroll
+        for (int h = 0; h < 2; ++h)   // C fragment: channel rows gid, gid + 8; pixel columns 2 tig, 2 tig + 1
+          *reinterpret_cast<float2*>(dst + (16 * i + gid + 8 * h) * c.ldr + 8 * j + 2 * tig) =
+              make_float2(acc[i][j][2 * h], acc[i][j][2 * h + 1]);
+  }
+  __syncthreads();
+  // ---- epilogue: k slices summed in order, bias, ReLU; one output channel's band is contiguous in y ----
+  const size_t ohw = (size_t)c.OH * c.OW;
+  float* yb = y + ((size_t)b * OC + oc0) * ohw + (size_t)y0 * c.OW;
+  for (int i = tid; i < CF_OC * npx; i += CF_T) {
+    const int oc = i / npx, p = i - oc * npx;
+    float v = red[oc * c.ldr + p];
+    for (int ks = 1; ks < c.ksplit; ++ks) v += red[((size_t)ks * CF_OC + oc) * c.ldr + p];
+    yb[(size_t)oc * ohw + p] = fmaxf(v + __ldg(bias + oc0 + oc), 0.0f);
+  }
+}
+
 int head_check(const rb_head_params* p, const char* who) {
   if (!p) return rbi::fail(RB_ERR_INVAL, who);
   for (int s = 0; s < 2; ++s)
@@ -1206,6 +1387,31 @@ int rb_conv_wgrad(const float* grad_out, const float* input, int B, int IC, int 
     k_conv_wgrad_reduce<<<(n_w + OC + CWR_J - 1) / CWR_J, 4 * CWR_J, 0, st>>>(partials, B * bands, n_w, OC, out, bias_out);
   }
   return rbi::check_launch("rb_conv_wgrad");
+}
+
+int rb_conv_forward(const float* input, const float* weight, const float* bias, int B, int IC, int IH, int IW, int OC, int K,
+                    int stride, float* out, rb_stream_t stream) {
+  if (!input || !weight || !bias || !out) return rbi::fail(RB_ERR_INVAL, "rb_conv_forward: null pointer");
+  if (B <= 0 || IC <= 0 || OC <= 0 || K <= 0 || stride <= 0 || IH < K || IW < K) return rbi::fail(RB_ERR_INVAL, "rb_conv_forward: bad shape");
+  const bool inst = (K == 8 && stride == 4) || (K == 4 && stride == 2) || (K == 3 && stride == 1) || (K == 5 && stride == 5);
+  if (!inst) return rbi::fail(RB_ERR_RANGE, "rb_conv_forward: (kernel, stride) in {(8,4), (4,2), (3,1), (5,5)} are instantiated");
+  if (OC % CF_OC) return rbi::fail(RB_ERR_RANGE, "rb_conv_forward: out_channels % 32 == 0 required");
+  const ConvFwdCfg c = conv_fwd_cfg(IC, IH, IW, K, stride);
+  if (c.smem > 200 * 1024) return rbi::fail(RB_ERR_RANGE, "rb_conv_forward: input band and weight rows do not fit in shared memory");
+  if (B > 65535) return rbi::fail(RB_ERR_RANGE, "rb_conv_forward: at most 65535 rows");
+  cudaStream_t st = (cudaStream_t)stream;
+  dim3 grid(c.bands, OC / CF_OC, B);
+  int rc = RB_OK;
+  {
+    rbi::ProfScope prof_(RB_K_CONV_FWD, st);
+#define RB_CF_LAUNCH(K_, S_)                                                                                           \
+  rc = rbi::ensure_dynamic_smem(k_conv_fwd<K_, S_>, c.smem, "rb_conv_forward");                                       \
+  if (rc == RB_OK) k_conv_fwd<K_, S_><<<grid, CF_T, c.smem, st>>>(input, weight, bias, IC, IH, IW, OC, c, out);
+    if (K == 8) { RB_CF_LAUNCH(8, 4) } else if (K == 4) { RB_CF_LAUNCH(4, 2) } else if (K == 3) { RB_CF_LAUNCH(3, 1) } else { RB_CF_LAUNCH(5, 5) }
+#undef RB_CF_LAUNCH
+  }
+  if (rc != RB_OK) return rc;
+  return rbi::check_launch("rb_conv_forward");
 }
 
 int rb_noise_factors(float* f_in, int n_in, float* f_out, int n_out, const float* x_in, const float* x_out, uint64_t seed,

@@ -4,7 +4,11 @@ API and state_dict layout follow the reference's model.py (NoisyLinear model.py:
 model.py:49-85) so checkpoints interchange: convs.{0,2,4}.{weight,bias} and
 fc_{h_v,h_a,z_v,z_a}.{weight_mu,weight_sigma,bias_mu,bias_sigma,weight_epsilon,bias_epsilon}.
 
-Per the north star the conv body stays a cuDNN torch forward.  What is ours:
+The conv body's parameters, layout, autograd path (features()) and backward stay torch / cuDNN.  What is ours:
+  * the conv body's forward on the learner, act and evaluation paths (conv_forward_saving / features_nograd): one
+    rb_conv_forward launch per layer (csrc/rb_head.cu k_conv_fwd, conv + bias + ReLU as an implicit GEMM on the tensor cores,
+    error-compensated TF32 = fp32-accurate whatever allow_tf32 says).  It replaced cuDNN's fused conv + ReLU, whose fp32
+    kernels were the largest block on the update's critical path and take as long at 64 rows as at 32;
   * noise lives as FACTOR VECTORS f(eps_in), f(eps_out) per layer (model.py:36-38); reset_noise() is one tiny
     rb_noise_factors launch (device Philox + Box-Muller) instead of the reference's ~52 ATen ops and 13.6 MB of
     weight_epsilon writes per net.  The weight_epsilon / bias_epsilon buffers of the state_dict are materialised
@@ -25,6 +29,8 @@ from torch import nn
 from torch.nn import functional as F
 
 from . import _lib
+
+RB_ERR_RANGE = -34   # include/rainbow_b200.h: shape outside what a kernel instantiates
 
 _ARCH = {
     # name: (conv specs (out_channels, kernel, stride), flattened conv output size)   model.py:55-63
@@ -314,12 +320,37 @@ class DQN(nn.Module):
     def manual_conv_ok(self, x):
         return x.is_cuda and torch.backends.cudnn.enabled
 
-    def conv_forward_saving(self, x):
-        """Conv body through cuDNN's fused conv + bias + ReLU, keeping every layer's input for the manual backward.
-        Returns [a0 = x, a1, ..., aL] (aL = ReLU(conv_L(...)), the conv features)."""
+    def _own_conv_body(self, x):
+        """[a0 = x, a1, ..., aL] through rb_conv_forward (csrc/rb_head.cu k_conv_fwd: conv + bias + ReLU, one launch per layer),
+        or None when the input is not a contiguous fp32 CUDA tensor or the kernel does not instantiate a layer's shape."""
+        if not (x.is_cuda and x.dtype == torch.float32 and x.is_contiguous() and x.dim() == 4):
+            return None
+        lib = _lib.load()
         acts = [x]
         for m in self.conv_layers():
-            acts.append(torch.cudnn_convolution_relu(acts[-1], m.weight, m.bias, m.stride, m.padding, m.dilation, m.groups))
+            a = acts[-1]
+            if (m.padding != (0, 0) or m.dilation != (1, 1) or m.groups != 1 or m.kernel_size[0] != m.kernel_size[1] or
+                    m.stride[0] != m.stride[1] or not (m.weight.is_contiguous() and m.bias.is_contiguous())):
+                return None
+            k, s = m.kernel_size[0], m.stride[0]
+            y = torch.empty((a.shape[0], m.out_channels, (a.shape[2] - k) // s + 1, (a.shape[3] - k) // s + 1),
+                            dtype=torch.float32, device=a.device)
+            rc = lib.rb_conv_forward(_lib.ptr(a), _lib.ptr(m.weight), _lib.ptr(m.bias), a.shape[0], a.shape[1], a.shape[2], a.shape[3],
+                                     m.out_channels, k, s, _lib.ptr(y), _lib.stream())
+            if rc == RB_ERR_RANGE:
+                return None
+            _lib.check(rc)
+            acts.append(y)
+        return acts
+
+    def conv_forward_saving(self, x):
+        """Conv body keeping every layer's input for the manual backward: [a0 = x, a1, ..., aL] (aL = ReLU(conv_L(...)), the
+        conv features).  Own tensor-core kernel per layer; shapes it does not cover go through the modules of features()."""
+        acts = self._own_conv_body(x)
+        if acts is None:
+            acts = [x]
+            for i in range(0, len(self.convs), 2):
+                acts.append(self.convs[i + 1](self.convs[i](acts[-1])))
         return acts
 
     def _own_wgrad_ok(self, m, a_in):
@@ -384,14 +415,12 @@ class DQN(nn.Module):
         return done
 
     def features_nograd(self, x):
-        """Inference-only conv body: cuDNN's fused conv + bias + ReLU (one launch per layer instead of three).
-        Same arithmetic as features() (bit-identical outputs on B200 [probe tools/conv_probe.py])."""
-        if not (x.is_cuda and torch.backends.cudnn.enabled):
+        """Inference-only conv body: the own conv + bias + ReLU kernel per layer (fp32-accurate, see _own_conv_body);
+        features() for inputs or shapes it does not cover."""
+        acts = self._own_conv_body(x)
+        if acts is None:
             return self.features(x)
-        for m in self.convs:
-            if isinstance(m, nn.Conv2d):
-                x = torch.cudnn_convolution_relu(x, m.weight, m.bias, m.stride, m.padding, m.dilation, m.groups)
-        return x.view(-1, self.conv_output_size)
+        return acts[-1].view(-1, self.conv_output_size)
 
     def logits(self, x):
         """Pre-softmax q [B, A, Z] (model.py:69-75)."""

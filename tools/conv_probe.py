@@ -1,12 +1,85 @@
-"""Probe (GPU): time library formulations of the canonical conv body at batch 32 inside CUDA graphs.
-Not part of the product; informs which torch/cuDNN configuration rainbow_b200.model uses."""
+"""Probe (GPU): time the conv body's forward inside CUDA graphs.
+First arm: the own kernel (rb_conv_forward) per layer at the learner's exact shapes -- online [s; s'] pass (64 rows, online
+weights), target pass (32 rows, target weights), canonical and data-efficient nets -- next to the same layer through cuDNN's
+fused conv + ReLU, with the achieved rate and the max |difference| against float64.  Then library formulations of the
+canonical body at batch B (argv[1], default 32).  Not part of the product; informs what rainbow_b200.model uses."""
+import argparse
+import os
 import sys
 import torch
 import torch.nn.functional as F
 
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+
 dev = "cuda"
 torch.manual_seed(0)
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 32
+torch.backends.cudnn.allow_tf32 = False
+FFMA_TFLOPS = 74.0   # 148 SMs x 128 FP32 lanes x 2 FLOP x 1.965 GHz: the plain-FFMA figure, not a tensor-core peak
+
+
+def graph_us(fn, reps=50, iters=20):
+    """Mean µs of one fn() call, replayed from a CUDA graph of `reps` calls (warm-up outside the graph)."""
+    for _ in range(3):
+        fn()
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        for _ in range(reps):
+            fn()
+    g.replay()
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(iters):
+        g.replay()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) * 1e3 / (iters * reps)
+
+
+def own_arm():
+    from rainbow_b200 import _lib
+    from rainbow_b200.model import DQN
+    lib = _lib.load()
+    print(f"{torch.cuda.get_device_name()}: own rb_conv_forward vs cuDNN cudnn_convolution_relu (fp32, allow_tf32=False), "
+          f"CUDA graphs; rate as a fraction of the {FFMA_TFLOPS:.0f} TFLOP/s plain-FFMA figure")
+    print(f"{'net':15s} {'pass':7s} {'rows':>4s} {'layer':24s} {'own us':>8s} {'cudnn us':>8s} {'GFLOP':>7s} "
+          f"{'own TFLOP/s':>11s} {'of FFMA':>7s} {'max|d| own':>10s} {'max|d| cudnn':>12s}")
+    for arch in ("canonical", "data-efficient"):
+        args = argparse.Namespace(device=torch.device(dev), history_length=4, atoms=51, architecture=arch, hidden_size=512,
+                                  noisy_std=0.1)
+        torch.manual_seed(1)
+        online = DQN(args, 6).to(dev)
+        torch.manual_seed(2)
+        target = DQN(args, 6).to(dev)
+        for pname, net, rows in (("online", online, 64), ("target", target, 32)):
+            x = torch.rand(rows, 4, 84, 84, device=dev)
+            tot_own = tot_cudnn = 0.0
+            for m in net.conv_layers():
+                k, s = m.kernel_size[0], m.stride[0]
+                oh = (x.shape[2] - k) // s + 1
+                y = torch.empty(rows, m.out_channels, oh, oh, device=dev)
+                args_ = (x.data_ptr(), m.weight.data_ptr(), m.bias.data_ptr(), rows, x.shape[1], x.shape[2], x.shape[3],
+                         m.out_channels, k, s, y.data_ptr())
+                own = graph_us(lambda: _lib.check(lib.rb_conv_forward(*args_, _lib.stream())))
+                ref_fn = lambda: torch.cudnn_convolution_relu(x, m.weight, m.bias, m.stride, m.padding, m.dilation, m.groups)
+                cud = graph_us(ref_fn)
+                with torch.no_grad():
+                    ref = F.relu(F.conv2d(x.double(), m.weight.double(), m.bias.double(), stride=s))
+                    d_own = float((y.double() - ref).abs().max())
+                    d_cud = float((ref_fn().double() - ref).abs().max())
+                flop = 2.0 * rows * m.out_channels * oh * oh * x.shape[1] * k * k
+                tflops = flop / (own * 1e-6) / 1e12
+                layer = f"{x.shape[1]}->{m.out_channels} k{k} s{s} {x.shape[2]}->{oh}"
+                print(f"{arch:15s} {pname:7s} {rows:4d} {layer:24s} {own:8.2f} {cud:8.2f} {flop / 1e9:7.3f} {tflops:11.2f} "
+                      f"{tflops / FFMA_TFLOPS:7.3f} {d_own:10.2e} {d_cud:12.2e}")
+                tot_own, tot_cudnn = tot_own + own, tot_cudnn + cud
+                x = y
+            print(f"{arch:15s} {pname:7s} {rows:4d} {'whole body (serial sum)':24s} {tot_own:8.2f} {tot_cudnn:8.2f}")
+
+
+own_arm()
 specs = [(4, 32, 8, 4), (32, 64, 4, 2), (64, 64, 3, 1)]
 ws = [torch.randn(co, ci, k, k, device=dev) * 0.05 for ci, co, k, s in specs]
 bs = [torch.randn(co, device=dev) * 0.05 for ci, co, k, s in specs]
