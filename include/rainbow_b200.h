@@ -185,7 +185,7 @@ int rb_noise_factors(float* f_in, int n_in, float* f_out, int n_out, const float
  * advantage (s=1) streams, W = mu + sigma * (eps_out (outer) eps_in) composed on the fly from the factor vectors
  * (model.py:39-44) -- weight_epsilon never has to exist in memory.  All pointers are device pointers; the eight
  * eps_* pointers are either all given (training mode) or all NULL (eval mode, model.py:45-46).
- * Requirements: conv_features % 32 == 0, hidden % 64 == 0. */
+ * Requirements: see rb_head_supported. */
 typedef struct rb_head_params {
   const float* w1_mu[2];    const float* w1_sigma[2];   /* [hidden][conv_features]        fc_h_v, fc_h_a */
   const float* b1_mu[2];    const float* b1_sigma[2];   /* [hidden] */
@@ -206,6 +206,11 @@ typedef struct rb_head_grads {   /* gradients are OVERWRITTEN (not accumulated) 
  * s1 is the larger of the two layer-1 implementations' factors (tensor-core kernel, csrc/rb_head_tc.cu; FFMA kernel). */
 int rb_head_splits(int conv_features, int hidden, int* s1, int* s2);
 int rb_head_ticket_count(void);
+/* RB_OK if rb_head_forward takes a head of this shape at `rows` rows and, with with_backward != 0, rb_head_backward takes it
+ * at a batch of `rows`; RB_ERR_RANGE for exactly the shapes those two refuse (conv_features % 32, hidden % 64,
+ * atoms <= RB_MAX_ATOMS, the forward's split-K tile count, B <= 32, the dh kernel's shared memory ~ actions * atoms <= 1065,
+ * hidden <= 1024).  Launches nothing; callers route the other shapes to the library path. */
+int rb_head_supported(int conv_features, int hidden, int atoms, int actions, int rows, int with_backward);
 /* probes / tests only: bit 0 skips the layer-1 launch of rb_head_forward, bit 1 the layer-2 launch, bit 2 forces the FFMA
  * layer-1 kernel instead of the tensor-core one (0 = normal) */
 int rb_head_debug(int flags);

@@ -47,6 +47,7 @@ SIGNATURES = {
     "rb_noise_factors": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _vp, _u64, _vp, _vp]),
     "rb_head_splits": (C.c_int, [_i32, _i32, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "rb_head_ticket_count": (C.c_int, []),
+    "rb_head_supported": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32]),
     "rb_head_debug": (C.c_int, [_i32]),
     "rb_head_forward": (C.c_int, [_hp, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rb_head_logits": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),

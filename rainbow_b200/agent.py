@@ -331,8 +331,11 @@ class Agent:
 
     # ---- the update ------------------------------------------------------------------------------
     def _fused_path(self, B):
+        """The fused head takes the update: online forward over [s; s'], target forward over s', backward over the batch
+        (B <= 32, and the head shape within the backward kernels' limits).  Everything else takes the library path."""
         on = self.online_net
-        return self.use_fused_head and B <= 32 and on.training and on.fused_ok(2 * B) and self.target_net.fused_ok(B)
+        return (self.use_fused_head and on.training and on.fused_ok(2 * B) and on.fused_ok(B, backward=True) and
+                self.target_net.fused_ok(B))
 
     @staticmethod
     def _adjacent(states, next_states):

@@ -513,6 +513,13 @@ k_head_wgrad2(const __grid_constant__ HeadDesc d, const __grid_constant__ HeadGr
 constexpr int DH_KB = 8;    // hidden units per CTA
 constexpr int DH_T = 256;   // 32 batch rows x 8 hidden units
 
+// the dz block [32][ld_dz] plus the mu and sigma slabs [Ns][DH_KB] of the wider stream
+int head_dh_ld(int Z, int A) { return (A * Z > Z ? A * Z : Z) | 1; }   // odd row stride: the 32 rows of a column hit 32 different banks
+size_t head_dh_smem(int Z, int A) {
+  const int ns_max = A * Z > Z ? A * Z : Z;
+  return ((size_t)32 * head_dh_ld(Z, A) + 2 * (size_t)((ns_max + 3) & ~3) * DH_KB) * sizeof(float);
+}
+
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(sa), "l"(gmem));
@@ -1189,8 +1196,25 @@ int head_check(const rb_head_params* p, const char* who) {
                            (uintptr_t)p->eps_out1[s] | (uintptr_t)p->eps_in2[s];
     if (bits & 15) return rbi::fail(RB_ERR_INVAL, "rb_head: weight / bias / factor pointers must be 16-byte aligned");
   }
-  if (p->conv_features % 32 || p->hidden % 64) return rbi::fail(RB_ERR_RANGE, "rb_head: conv_features % 32 == 0 and hidden % 64 == 0 required");
   return RB_OK;
+}
+
+// Every shape limit of the head kernels, in one place: nullptr if a forward over `rows` rows (and, with `with_backward`,
+// the backward over a batch of `rows`) launches, else why not.  rb_head_forward / rb_head_backward refuse exactly these
+// shapes, and rb_head_supported lets a caller route them to the library path before it launches anything.
+const char* head_limit(int K1, int H, int Z, int A, int rows, bool with_backward) {
+  if (K1 % 32 || H % 64) return "rb_head: conv_features % 32 == 0 and hidden % 64 == 0 required";
+  if (Z > RB_MAX_ATOMS) return "rb_head: atoms exceeds RB_MAX_ATOMS";
+  // forward: one split-K ticket per (row tile, column tile) of each layer, 2048 tickets per layer
+  const int MT = (rows > 32) ? 64 : 32;
+  const int mt = (rows + MT - 1) / MT;
+  const int tiles1 = 2 * H / NT, tiles2 = (Z + NT - 1) / NT + (A * Z + NT - 1) / NT;
+  if (mt > 65535 || mt * tiles1 > 2048 || mt * tiles2 > 2048) return "rb_head_forward: too many rows for this head shape";
+  if (!with_backward) return nullptr;
+  if (rows > 32) return "rb_head_backward: 1 <= B <= 32 required (larger batches use the library GEMM path)";
+  if (head_dh_smem(Z, A) > 200 * 1024) return "rb_head_backward: actions * atoms too large for the dh kernel";
+  if (H > 1024) return "rb_head_backward: hidden <= 1024 required";
+  return nullptr;
 }
 
 void head_splits(int K1, int H, int* s1, int* s2, int* ks1, int* ks2) {
@@ -1227,6 +1251,12 @@ int rb_head_splits(int conv_features, int hidden, int* s1, int* s2) {
 
 int rb_head_ticket_count(void) { return 4096; }
 
+int rb_head_supported(int conv_features, int hidden, int atoms, int actions, int rows, int with_backward) {
+  if (conv_features <= 0 || hidden <= 0 || atoms <= 1 || actions <= 0 || rows <= 0)
+    return rbi::fail(RB_ERR_INVAL, "rb_head_supported: bad argument");
+  return head_limit(conv_features, hidden, atoms, actions, rows, with_backward != 0) ? RB_ERR_RANGE : RB_OK;
+}
+
 static int g_head_debug = 0;   // bit 0: skip the layer-1 launch, bit 1: skip the layer-2 launch (timing probes only); bit 2: FFMA layer 1; bit 3: split-K layer 2
 int rb_head_debug(int flags) {
   g_head_debug = flags;
@@ -1241,13 +1271,13 @@ int rb_head_forward(const rb_head_params* p, const float* x_lo, int m_lo, const 
   if (!x_lo || m_lo <= 0 || m_hi < 0 || (m_hi > 0 && !x_hi) || !part1 || !part2 || !tickets || !h || !z)
     return rbi::fail(RB_ERR_INVAL, "rb_head_forward: bad argument");
   const HeadDesc d = to_desc(p);
+  if (const char* why = head_limit(d.K1, d.H, d.Z, d.A, M, false)) return rbi::fail(RB_ERR_RANGE, why);
   int s1, s2, ks1, ks2;
   head_splits(d.K1, d.H, &s1, &s2, &ks1, &ks2);
   cudaStream_t st = (cudaStream_t)stream;
   const int MT = (M > 32) ? 64 : 32;
   const int mt = (M + MT - 1) / MT;
   const int tiles1 = 2 * d.H / NT, tiles2 = (d.Z + NT - 1) / NT + (d.A * d.Z + NT - 1) / NT;
-  if (mt > 65535 || mt * tiles1 > 2048 || mt * tiles2 > 2048) return rbi::fail(RB_ERR_RANGE, "rb_head_forward: too many rows");
   const size_t smem64 = (size_t)FC_STAGES * (64 + 2 * NT) * (KT + 4) * sizeof(float);
   const size_t smem32 = (size_t)FC_STAGES * (32 + 2 * NT) * (KT + 4) * sizeof(float);
   rc = rbi::ensure_dynamic_smem(k_head_fc<64, 1>, smem64, "rb_head_forward");
@@ -1300,7 +1330,10 @@ int rb_head_backward(const rb_head_params* p, const rb_head_grads* gr, const flo
   if ((parts & 7) == 0) return rbi::fail(RB_ERR_INVAL, "rb_head_backward: parts must select at least one of RB_HEAD_BWD_*");
   if (rc != RB_OK) return rc;
   if (!gr || !x || !h || !dz || !dh_scratch || !dx) return rbi::fail(RB_ERR_INVAL, "rb_head_backward: null pointer");
-  if (B <= 0 || B > 32) return rbi::fail(RB_ERR_RANGE, "rb_head_backward: 1 <= B <= 32 required (larger batches use the library GEMM path)");
+  if (B <= 0) return rbi::fail(RB_ERR_RANGE, "rb_head_backward: 1 <= B <= 32 required");
+  // the whole backward's limits, whichever parts this call enqueues: a shape never gets its layer-2 gradient on one stream
+  // and a refusal of the dh / layer-1 launches on the other
+  if (const char* why = head_limit(p->conv_features, p->hidden, p->atoms, p->actions, B, true)) return rbi::fail(RB_ERR_RANGE, why);
   HeadGrads g;
   for (int s = 0; s < 2; ++s) {
     if (!gr->w1_mu[s] || !gr->w1_sigma[s] || !gr->b1_mu[s] || !gr->b1_sigma[s] || !gr->w2_mu[s] || !gr->w2_sigma[s] ||
@@ -1320,10 +1353,8 @@ int rb_head_backward(const rb_head_params* p, const rb_head_grads* gr, const flo
   rc = rbi::check_launch("rb_head_backward(wgrad2)");
   if (rc != RB_OK) return rc;
   if (parts & RB_HEAD_BWD_DH) {
-    const int ns_max = d.A * d.Z > d.Z ? d.A * d.Z : d.Z;
-    const int ld_dz = ns_max | 1;                       // odd row stride: the 32 rows of a column hit 32 different banks
-    const size_t smem = ((size_t)32 * ld_dz + 2 * (size_t)((ns_max + 3) & ~3) * DH_KB) * sizeof(float);
-    if (smem > 200 * 1024 || d.H % DH_KB) return rbi::fail(RB_ERR_RANGE, "rb_head_backward: actions * atoms too large for the dh kernel");
+    const int ld_dz = head_dh_ld(d.Z, d.A);
+    const size_t smem = head_dh_smem(d.Z, d.A);
     rc = rbi::ensure_dynamic_smem(k_head_dh, smem, "rb_head_backward");
     if (rc != RB_OK) return rc;
     dim3 grid(d.H / DH_KB, 2);
@@ -1333,7 +1364,6 @@ int rb_head_backward(const rb_head_params* p, const rb_head_grads* gr, const flo
   rc = rbi::check_launch("rb_head_backward(dh)");
   if (rc != RB_OK) return rc;
   if (parts & RB_HEAD_BWD_LAYER1) {
-    if (d.H > 1024) return rbi::fail(RB_ERR_RANGE, "rb_head_backward: hidden <= 1024 required");
     dim3 grid(d.K1 / B1_K, 4);
     rbi::ProfScope prof_(RB_K_HEAD_BWD1, st);
     const size_t smem_b1 = (size_t)B1_STAGES * B1_STAGE * sizeof(float);

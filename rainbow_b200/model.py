@@ -112,9 +112,16 @@ class FusedHead:
         self._tickets = None
 
     @staticmethod
-    def supported(net):
-        return (net.conv_output_size % 32 == 0 and net.hidden_size % 64 == 0 and net.atoms <= 128 and
-                next(net.parameters()).is_cuda)
+    def supported(net, rows, backward=False):
+        """Whether the kernels take this net's head at `rows` rows (and, with `backward`, its backward at a batch of `rows`):
+        the library's own limits (rb_head_supported), so a shape they refuse is routed elsewhere instead of raising."""
+        if not next(net.parameters()).is_cuda:
+            return False
+        rc = _lib.load().rb_head_supported(net.conv_output_size, net.hidden_size, net.atoms, net.action_space, rows,
+                                           1 if backward else 0)
+        if rc not in (0, RB_ERR_RANGE):
+            _lib.check(rc)
+        return rc == 0
 
     def params(self, noisy=None):
         net = self.net
@@ -307,8 +314,8 @@ class DQN(nn.Module):
             self._head = FusedHead(self)
         return self._head
 
-    def fused_ok(self, rows):
-        return self.use_fused_head and rows <= FusedHead.MAX_ROWS and FusedHead.supported(self)
+    def fused_ok(self, rows, backward=False):
+        return self.use_fused_head and rows <= FusedHead.MAX_ROWS and FusedHead.supported(self, rows, backward)
 
     def features(self, x):
         return self.convs(x).view(-1, self.conv_output_size)
